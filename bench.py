@@ -7,6 +7,7 @@ candidates passes the confidence filter and the 300-detection cap is hit.
 
   python bench.py [--gpus N --steps K --warmup W]          our CUDA path (one process per GPU under torchrun)
   python bench.py --impl reference ...                      the CPU restatement of the reference (oracle/) on host cores
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step computed as DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  `value` = whole-job images/s with inputs resident in HBM; `e2e` = the same
 through yfv2_detect_u8_host with pinned HOST uint8 images in and pinned HOST detections out, copies inside the
@@ -32,6 +33,7 @@ CONF, IOU = 0.001, 0.4
 METRIC = "images/sec 352x352 fwd+decode+NMS"
 UNIT_NAMES = (["stem"] + ["stage2.%d" % i for i in range(4)] + ["stage3.%d" % i for i in range(8)]
               + ["stage4.%d" % i for i in range(4)] + ["fpn.S3", "fpn.S2", "heads2.a", "heads2.b", "heads3.a", "heads3.b"])
+DUMP_BYTES = 64_000_000 - 4096      # --dump-outputs: all .npy files together (headers included) stay under 64 MB
 
 
 def cfg():
@@ -250,6 +252,32 @@ def parity_check(model, x, preds, out, counts, c, dev, n=8):
             "fused_equals_unfused": True}
 
 
+def dump_outputs(d, preds, out, counts):
+    """Writes what a caller of the timed path holds after its last step, as d/<name>.npy: the six head tensors
+    (reg_s16, obj_s16, cls_s16, reg_s32, obj_s32, cls_s32; float32 NCHW), the detections [N,300,6] (float32; rows past
+    counts[i] are not part of the result and are written as zeros) and counts [N] (float64).  image_index.npy (float64) lists
+    the batch positions written: all of them, or a fixed seeded subset when the whole batch would exceed DUMP_BYTES."""
+    import numpy as np
+    arrays = {}
+    for lv, s in enumerate((16, 32)):
+        for j, nm in enumerate(("reg", "obj", "cls")):
+            arrays["%s_s%d" % (nm, s)] = preds[3 * lv + j]
+    valid = torch.arange(out.shape[1], device=out.device)[None, :] < counts[:, None]
+    arrays["detections"] = torch.where(valid[:, :, None], out, torch.zeros((), dtype=out.dtype, device=out.device))
+    arrays["counts"] = counts.double()
+    n = counts.shape[0]
+    per_image = sum(a[0].numel() * a.element_size() for a in arrays.values()) + 8
+    idx = torch.arange(n)
+    if per_image * n > DUMP_BYTES:
+        k = max(1, DUMP_BYTES // per_image)
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a[idx.to(a.device)].cpu().numpy())
+    np.save(os.path.join(d, "image_index.npy"), idx.double().numpy())
+    return len(idx)
+
+
 # ------------------------------------------------------------------------------------------------------------
 def run_ours(args, rank, world, local_rank):
     import yfv2  # noqa: F401
@@ -317,6 +345,10 @@ def run_ours(args, rank, world, local_rank):
     ms = float(t.item())
     value = world * BATCH * args.steps / (ms / 1e3)
     kept = int(counts.sum().item())
+    if args.dump_outputs and rank == 0:                       # before anything below reuses preds / out / counts
+        k = dump_outputs(args.dump_outputs, preds, out, counts)
+        print("bench.py: wrote the outputs of timed step %d (%d of %d images) to %s" % (args.steps, k, BATCH, args.dump_outputs),
+              file=sys.stderr)
 
     # ---- parity of THIS workload (outside the timed region): first images of the step against the CPU oracle ---------
     parity = None
@@ -606,7 +638,14 @@ def main():
     ap.add_argument("--batch", type=int, default=256, help="images per GPU")
     ap.add_argument("--input", default="u8", choices=["u8", "f32"], help="dtype of the HBM-resident input batch of the device-timed step")
     ap.add_argument("--mode", default="infer", choices=["infer", "train"], help="infer: BASELINE configs[1] (default); train: configs[2]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (head tensors, detections, counts; rank 0) as DIR/<name>.npy. "
+                         "Inputs and weights are seeded, so the same arguments give the same inputs on every run and build")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs applies to the inference workload of --impl ours")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

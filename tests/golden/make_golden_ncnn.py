@@ -1,7 +1,8 @@
 """Golden vectors for the deploy post-process (SURVEY 8f.4): outputs of the REFERENCE's own C++ (sample/ncnn/src/yolo-fastestv2.cpp
 predHandle + nmsHandle, compiled in place by `make -C oracle ref` against stub ncnn/OpenCV headers) on export_onnx head tensors.
+Writes ncnn_post.npz and ncnn_post_fresh.npz (same layout, other seeds and shape).
 
-Run in the build container (needs /root/reference):  python tests/golden/make_golden_ncnn.py
+Run where the reference checkout is available (oracle/Makefile REF):  python tests/golden/make_golden_ncnn.py
 Inputs are stored in the .npz (not regenerated) so the fixture does not depend on the host's exp()/sigmoid code paths.
 """
 import ctypes
@@ -57,7 +58,22 @@ def no_ties(o2, o3, A, thresh):
     return len(np.unique(sc)) == len(sc)
 
 
-out = {}
+def save(fname, cases):
+    out = {}
+    for (name, o2, o3, A, C, iw, ih, anc, thr, nms, sw, sh) in cases:
+        assert no_ties(o2, o3, A, thr), name
+        b, s, c = run_ref(np.ascontiguousarray(o2), np.ascontiguousarray(o3), A, C, iw, ih, anc, thr, nms, sw, sh)
+        print(name, "kept", len(s), "top", s[:3], c[:3])
+        out[name + "_out2"] = o2; out[name + "_out3"] = o3
+        out[name + "_params"] = np.array([A, C, iw, ih, sw, sh], np.int32)
+        out[name + "_fparams"] = np.array([thr, nms], np.float32)
+        out[name + "_anchors"] = anc
+        out[name + "_boxes"] = b; out[name + "_scores"] = s; out[name + "_cates"] = c
+    out["names"] = np.array([c[0] for c in cases])
+    np.savez_compressed(os.path.join(HERE, fname), **out)
+    print("wrote", os.path.join(HERE, fname), os.path.getsize(os.path.join(HERE, fname)), "bytes")
+
+
 cases = []
 zoo = np.load(os.path.join(HERE, "images_modelzoo.npz"))
 # 1-2: the bundled images through the modelzoo weights (352x352), the sample's defaults (thresh 0.3, NMS 0.25) and a low threshold;
@@ -77,15 +93,15 @@ p = list(synth.make_head_logits(32, 1, 320, 256, classes=5, anchor_num=2, obj_me
 o2, o3 = export_heads(p)
 anc = np.array([10, 14, 40, 60, 90, 70, 200, 180], np.float32)
 cases.append(("a2c5_320x256", o2[0], o3[0], 2, 5, 256, 320, anc, 0.05, 0.45, 1024, 960))
-for (name, o2, o3, A, C, iw, ih, anc, thr, nms, sw, sh) in cases:
-    assert no_ties(o2, o3, A, thr), name
-    b, s, c = run_ref(np.ascontiguousarray(o2), np.ascontiguousarray(o3), A, C, iw, ih, anc, thr, nms, sw, sh)
-    print(name, "kept", len(s), "top", s[:3], c[:3])
-    out[name + "_out2"] = o2; out[name + "_out3"] = o3
-    out[name + "_params"] = np.array([A, C, iw, ih, sw, sh], np.int32)
-    out[name + "_fparams"] = np.array([thr, nms], np.float32)
-    out[name + "_anchors"] = anc
-    out[name + "_boxes"] = b; out[name + "_scores"] = s; out[name + "_cates"] = c
-out["names"] = np.array([c[0] for c in cases])
-np.savez_compressed(os.path.join(HERE, "ncnn_post.npz"), **out)
-print("wrote", os.path.join(HERE, "ncnn_post.npz"), os.path.getsize(os.path.join(HERE, "ncnn_post.npz")), "bytes")
+save("ncnn_post.npz", cases)
+
+# ncnn_post_fresh.npz: seeds that ncnn_post.npz does not use, at 224x160 input, 3 anchors, 80 classes, two dominant classes,
+# thresh 0.01, NMS 0.3, source 448x320 (scale 2).  Three seeds keep the fixture small (~190 KB; the inputs are incompressible).
+fresh = []
+for seed in (40, 41, 42):
+    p = list(synth.make_head_logits(seed, 1, 160, 224, obj_mean=-0.5))
+    for i in (2, 5):
+        p[i][:, :2] += 5.0
+    o2, o3 = export_heads(p)
+    fresh.append(("seed%d_224x160" % seed, o2[0], o3[0], 3, 80, 224, 160, COCO, 0.01, 0.3, 448, 320))
+save("ncnn_post_fresh.npz", fresh)

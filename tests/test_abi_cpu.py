@@ -82,21 +82,33 @@ def test_load_datafile(tmp_path):
                         "classes", "width", "height", "anchor_num", "anchors", "val", "train", "names"}
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/utils"), reason="reference checkout not present (build container only)")
-def test_overlay_resolves_out_of_scope_names_from_the_reference():
-    """With the reference checkout behind the mirror on sys.path, utils.datasets / utils.utils.evaluation come from the
-    reference while the hot-path functions stay ours (what train.py / evaluation.py need to run unchanged)."""
+def test_overlay_resolves_out_of_scope_names_from_the_reference(tmp_path, golden_dir):
+    """With a reference checkout behind the mirror on sys.path, utils.datasets and the utils.utils names the mirror does not define
+    come from the reference while the hot-path functions stay ours (what train.py / evaluation.py need to run unchanged).  The
+    checkout is a stub with the reference's layout whose modules define the public names the real ones do
+    (golden/reference_names.json, make_golden_names.py)."""
     import subprocess, sys as _sys, textwrap
+    names = json.load(open(os.path.join(golden_dir, "reference_names.json")))
+    ref = tmp_path / "reference"
+    for d in ("utils", "model"):
+        (ref / d).mkdir(parents=True)
+    for rel, defined in names.items():
+        (ref / rel).write_text("".join("def %s(*a, **k):\n    return 'reference'\n" % n for n in defined))
+    for rel in ("utils/loss.py", "model/detector.py"):              # the mirror must shadow these
+        (ref / rel).write_text("raise ImportError('the reference module was imported instead of the mirror')\n")
     code = textwrap.dedent("""
-        import sys, types
-        ts = types.ModuleType("torchsummary"); ts.summary = lambda *a, **k: None; sys.modules["torchsummary"] = ts
-        sys.path.insert(0, "/root/reference"); sys.path.insert(0, "%s")
+        import sys
+        mirror, ref, utils_names, dataset_names = %r, %r, %r, %r
+        sys.path.insert(0, ref); sys.path.insert(0, mirror)
         import utils.utils as uu, utils.datasets as ud, utils.loss as ul, model.detector as md
-        assert "yolo-fastestv2_b200" in uu.__file__ and "yolo-fastestv2_b200" in ul.__file__ and "yolo-fastestv2_b200" in md.__file__
-        assert ud.__file__.startswith("/root/reference") and hasattr(ud, "TensorDataset") and hasattr(ud, "collate_fn")
+        assert uu.__file__.startswith(mirror) and ul.__file__.startswith(mirror) and md.__file__.startswith(mirror)
+        assert ud.__file__.startswith(ref) and all(getattr(ud, n)() == "reference" for n in dataset_names)
+        src = {n: getattr(uu, n).__module__ for n in utils_names}
+        assert src.pop("make_grid") == "_yfv2_reference_utils", "make_grid not taken from the reference"
+        assert set(src.values()) == {"utils.utils"}, src          # every other name the reference defines, the mirror defines itself
         assert callable(uu.evaluation) and uu.evaluation.__globals__["non_max_suppression"] is uu.non_max_suppression
         print("ok")
-    """ % os.path.join(ROOT, "yolo-fastestv2_b200"))
+    """ % (os.path.join(ROOT, "yolo-fastestv2_b200"), str(ref), names["utils/utils.py"], names["utils/datasets.py"]))
     r = subprocess.run([_sys.executable, "-c", code], capture_output=True, text=True)
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
 
