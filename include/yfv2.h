@@ -146,6 +146,19 @@ YFV2_API int yfv2_batch_statistics(const float* dets, const int* counts, int N, 
 YFV2_API int yfv2_aug_contrast_brightness(const uint8_t* img, uint8_t* out, const float* alpha, const float* beta, int N,
                                           long long bytes_per_image, void* stream);
 
+/* ---- cv2.resize(img, (W, H), interpolation=cv2.INTER_LINEAR) + transpose(2,0,1) on the device -------------------------------
+ * The first step of every input path of the reference: utils/datasets.py:106-111 (TensorDataset.__getitem__, behind train.py
+ * and evaluation()) and test.py:34-37, both right after cv2.imread.  src: HOST array of N device pointers, one HWC uint8 image
+ * each (3 channels, rows contiguous: 3*w bytes; any byte alignment); src_hw: HOST array [N][2] of (h, w).  out: device uint8
+ * [N,3,H,W], the input of yfv2_forward_u8; channel order is kept.  Bit-identical to OpenCV 4.x's uint8 INTER_LINEAR (its fixed-
+ * point coefficients and rounding, incl. the exact 2x / 3x downscales it routes through INTER_AREA).  Both host arrays are read
+ * before the call returns (the descriptors travel in kernel parameters, 256 images per launch).  Arguments are checked before
+ * any launch: null pointers, N <= 0, an empty size or `out` overlapping a source give YFV2_EINVAL, sizes above the limits
+ * below YFV2_EUNSUPPORTED. */
+#define YFV2_RESIZE_MAX_SRC 8192   /* source h, w */
+#define YFV2_RESIZE_MAX_DST 1024   /* destination H, W */
+YFV2_API int yfv2_resize_u8(const uint8_t* const* src, const int* src_hw, int N, int H, int W, uint8_t* out, void* stream);
+
 /* ---- whole inference step with HOST buffers (the evaluation() inner loop, utils/utils.py:367-383) ----
  * x_host: pinned uint8 [N,3,H,W]; out_host: pinned [N,max_det,6]; counts_host: pinned [N].
  * Copies in, runs forward_u8 + decode_nms, copies out, all on `stream`; returns without synchronising. */

@@ -55,6 +55,17 @@ class SyntheticDetection(torch.utils.data.Dataset):
         return img, t
 
 
+class SyntheticRawDetection(SyntheticDetection):
+    """Decoded-image form of SyntheticDetection for --device-resize: uint8 HWC images of seeded sizes (as cv2.imread returns
+    them, before any resize) with the same kind of label rows."""
+
+    def __getitem__(self, i):
+        g = torch.Generator().manual_seed(self.seed * 1000003 + i)
+        h, w = int(torch.randint(96, 641, (1,), generator=g)), int(torch.randint(96, 641, (1,), generator=g))
+        _, t = super().__getitem__(i)
+        return torch.randint(0, 256, (h, w, 3), generator=g, dtype=torch.uint8), t
+
+
 def collate_fn(batch):
     """utils/datasets.py:127-135: image index into column 0, targets concatenated."""
     imgs, targets = list(zip(*batch))
@@ -72,6 +83,9 @@ def main(argv=None):
     ap.add_argument("--save-dir", type=str, default="weights")
     ap.add_argument("--device-aug", action="store_true", help="run contrast_and_brightness (utils/datasets.py:10-16) on the uint8 batch "
                                                               "on the GPU (csrc/k_aug.cu) instead of per image in the data-loader workers")
+    ap.add_argument("--device-resize", action="store_true", help="data-loader workers only decode; the cv2.resize of "
+                                                                 "utils/datasets.py:106-111 runs on the GPU (csrc/k_resize.cu), followed by "
+                                                                 "contrast_and_brightness for the training batches")
     opt = ap.parse_args(argv)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -93,7 +107,15 @@ def main(argv=None):
 
     batch_size = int(cfg["batch_size"] / cfg["subdivisions"])                     # per rank, as train.py:37
     nw = min([os.cpu_count(), batch_size if batch_size > 1 else 0, 8])
-    if opt.synthetic:
+    if opt.device_resize:
+        import utils.device_aug
+        cf = utils.device_aug.collate_packed
+        if opt.synthetic:
+            train_dataset, val_dataset = SyntheticRawDetection(opt.synthetic, cfg["width"], cfg["height"], cfg["classes"]), None
+        else:
+            train_dataset = utils.device_aug.RawImageDataset(cfg["train"], cfg["width"], cfg["height"])
+            val_dataset = utils.device_aug.RawImageDataset(cfg["val"], cfg["width"], cfg["height"])
+    elif opt.synthetic:
         train_dataset = SyntheticDetection(opt.synthetic, cfg["width"], cfg["height"], cfg["classes"])
         val_dataset, cf = None, collate_fn
     else:
@@ -108,6 +130,12 @@ def main(argv=None):
     if val_dataset is not None and rank == 0:
         val_dataloader = DataLoader(val_dataset, batch_size=batch_size, shuffle=False, collate_fn=cf, num_workers=nw,
                                     pin_memory=True, drop_last=False, persistent_workers=nw > 0)
+    if opt.device_resize:
+        # the reference augments every training image (train.py: TensorDataset(..., imgaug=True)); synthetic data only with --device-aug
+        train_dataloader = utils.device_aug.DeviceResizeLoader(train_dataloader, cfg["width"], cfg["height"], device,
+                                                               imgaug=opt.device_aug or not opt.synthetic)
+        if val_dataloader is not None:
+            val_dataloader = utils.device_aug.DeviceResizeLoader(val_dataloader, cfg["width"], cfg["height"], device)
 
     load_param = bool(cfg["pre_weights"]) and os.path.exists(cfg["pre_weights"])
     torch.manual_seed(0)                                                          # identical initial weights on every rank
@@ -133,7 +161,7 @@ def main(argv=None):
         sampler.set_epoch(epoch)
         for imgs, targets in train_dataloader:
             imgs = imgs.to(device, non_blocking=True)
-            if opt.device_aug and imgs.dtype == torch.uint8:
+            if opt.device_aug and not opt.device_resize and imgs.dtype == torch.uint8:   # (DeviceResizeLoader augments itself)
                 import utils.device_aug
                 imgs = utils.device_aug.img_aug_batch(imgs, out=imgs)                 # datasets.py:63-68 on the device, in place
             imgs = imgs.float() / 255.0                                           # train.py:101

@@ -53,6 +53,8 @@ PROTOTYPES = {
     "yfv2_batch_statistics": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
                                              ctypes.c_int, ctypes.c_float, ctypes.c_void_p, ctypes.c_void_p]),
     "yfv2_aug_contrast_brightness": (ctypes.c_int, [ctypes.c_void_p] * 4 + [ctypes.c_int, ctypes.c_longlong, ctypes.c_void_p]),
+    "yfv2_resize_u8": (ctypes.c_int, [_c_void_pp, ctypes.POINTER(ctypes.c_int), ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                      ctypes.c_void_p, ctypes.c_void_p]),
     "yfv2_detect_u8_host": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                            ctypes.POINTER(ctypes.c_double), ctypes.c_float, ctypes.c_double, ctypes.c_int,
                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
@@ -439,6 +441,32 @@ def contrast_and_brightness(imgs, alpha, beta, out=None):
         _check(lib().yfv2_aug_contrast_brightness(ctypes.c_void_p(imgs.data_ptr()), ctypes.c_void_p(out.data_ptr()),
                                                   ctypes.c_void_p(alpha.data_ptr()), ctypes.c_void_p(beta.data_ptr()), N,
                                                   imgs.numel() // N, _stream(imgs.device)), "aug_contrast_brightness")
+    return out
+
+
+def resize_u8(images, height, width, out=None):
+    """cv2.resize(img, (width, height), interpolation=cv2.INTER_LINEAR) + transpose(2,0,1) for a batch on the device
+    (utils/datasets.py:106-111, test.py:34-37): images is a list of CUDA uint8 [h,w,3] tensors of any sizes (rows contiguous; views
+    at any byte offset are fine).  Returns CUDA uint8 [N,3,height,width] (or writes `out`)."""
+    images = list(images)
+    if not images:
+        raise ValueError("resize_u8: no images")
+    for im in images:
+        _require_cuda(im, "images")
+        if im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != 3:
+            raise Yfv2Error("resize_u8: images must be uint8 [h, w, 3], got %s %s" % (im.dtype, tuple(im.shape)))
+        if im.stride() != (3 * im.shape[1], 3, 1):
+            raise Yfv2Error("resize_u8: image rows must be contiguous")
+    dev = images[0].device
+    N = len(images)
+    if out is None:
+        out = torch.empty((N, 3, height, width), dtype=torch.uint8, device=dev)
+    elif tuple(out.shape) != (N, 3, height, width) or out.dtype != torch.uint8 or not out.is_contiguous() or out.device != dev:
+        raise Yfv2Error("resize_u8: out must be a contiguous uint8 [%d,3,%d,%d] tensor on %s" % (N, height, width, dev))
+    hw = (ctypes.c_int * (2 * N))(*[int(v) for im in images for v in im.shape[:2]])
+    with torch.cuda.device(dev):
+        _check(lib().yfv2_resize_u8(_ptr_array(images), hw, N, height, width, ctypes.c_void_p(out.data_ptr()), _stream(dev)),
+               "resize_u8")
     return out
 
 
